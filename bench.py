@@ -487,6 +487,8 @@ def bench_b200(args, rank, world, local_rank):
         launches = ctx.launches - l0
         ms = ev0.elapsed_time(ev1)
         graphs = pipe.graph_stats()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, pipe)
         # The dominant kernel's launch duration (roofline.achieved): CUDA events around the fused front-end launch of every
         # step of a SECOND pass of the same K steps, launched kernel by kernel -- the timed pass above replays CUDA graphs,
         # which cannot carry per-launch event pairs.  Same kernel, same inputs, same stream, right after the timed pass.
@@ -618,6 +620,20 @@ def bench_b200(args, rank, world, local_rank):
     print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, pipe):
+    """What the last timed step left for its caller -- the arrays alva_pipeline_step_host copies out: selected-feature counts
+    per frame, the 2-NN match lists, the local-BA poses and solver summaries -- as out_dir/<name>.npy (float64: exact for the
+    int32 arrays).  The inputs are seeded, so two builds run with the same arguments can be compared array by array."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"nfeat": pipe.buffer("selcounts", (BATCH,), torch.int32),
+              "matches": pipe.buffer("matches", (BATCH, pipe.fcap, 4), torch.int32),
+              "ba_poses": pipe.buffer("ba_poses", (pipe.nprob, BA_NKF, 7), torch.float64),
+              "ba_summary": pipe.buffer("ba_summary", (pipe.nprob, 8), torch.float64)}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float64))
 
 
 def print_checksums():
@@ -862,6 +878,7 @@ def main():
     ap.add_argument("--frontend-ctas", type=int, default=0, help="A/B: resident front-end CTAs per SM (4 | 5)")
     ap.add_argument("--ba-ctl-threads", type=int, default=0, help="A/B: CTA size of the BA control kernels (256 | 512 | 1024)")
     ap.add_argument("--no-graphs", action="store_true", help="launch kernel by kernel instead of replaying CUDA graphs (profiling aid)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
     select_config(args.config)
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup

@@ -6,7 +6,7 @@ import subprocess
 
 import numpy as np
 
-from conftest import P, ROOT, golden
+from conftest import P, ROOT, digest, golden
 from alvaar_b200 import synth
 
 CAP = 4096
@@ -43,6 +43,87 @@ def cpu_system_lib():
     S.cpu_system_set_essential_hook.argtypes = [C.c_void_p, C.c_void_p]
     S.cpu_system_destroy.argtypes = [C.c_void_p]
     return S
+
+
+_ESSENTIAL_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_int, C.c_float, C.c_float,
+                            C.c_void_p, C.c_void_p)
+
+
+class ReferenceEssential:
+    """The reference's compute5ptEssentialMatrix as the state machine's essential-matrix hook (`ptr`, for
+    cpu_system_set_essential_hook): ref_essential_5pt itself when the reference is built, else its recorded results, call by
+    call -- a call whose inputs (hashed) are not the recorded call's fails.  `finish()` records the calls, or checks that every
+    recorded call was made."""
+
+    def __init__(self, ref_results, key):
+        self.res, self.key, self.ref = ref_results, key, ref_results.lib
+        self.calls, self.mismatch = [], None
+        if self.ref is None:
+            self.want = ref_results.get(key, None)
+        else:
+            self.ref.ref_essential_5pt.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_int, C.c_float, C.c_float,
+                                                   C.c_void_p, C.c_void_p]
+        self.fn = _ESSENTIAL_FN(self._call)
+        self.ptr = C.cast(self.fn, C.c_void_p)
+
+    def _call(self, b1, b2, n, max_iter, err, opt, fx, fy, Rt, outl):
+        args = np.array([n, max_iter, opt], np.int32).tobytes() + np.array([err, fx, fy], np.float32).tobytes()
+        inputs = np.frombuffer(hashlib.sha256(C.string_at(b1, 24 * n) + C.string_at(b2, 24 * n) + args).digest(), np.uint8)
+        k = len(self.calls)
+        if self.ref is not None:
+            ok = self.ref.ref_essential_5pt(b1, b2, n, max_iter, err, opt, fx, fy, Rt, outl)
+        else:
+            digests, oks, Rts, outls, starts = self.want
+            if k >= len(oks) or (digests[k] != inputs).any():
+                self.mismatch = self.mismatch if self.mismatch is not None else k
+                return 0
+            ok = int(oks[k])
+            C.memmove(Rt, np.ascontiguousarray(Rts[k]).ctypes.data, 96)
+            C.memmove(outl, outls[starts[k]:starts[k + 1]].ctypes.data, n)
+        self.calls.append((inputs, ok, np.frombuffer(C.string_at(Rt, 96), np.float64), np.frombuffer(C.string_at(outl, n), np.uint8)))
+        return ok
+
+    def finish(self):
+        if self.ref is not None:
+            self.res.get(self.key, lambda: (np.array([c[0] for c in self.calls], np.uint8).reshape(-1, 32),
+                                            np.array([c[1] for c in self.calls], np.int32),
+                                            np.array([c[2] for c in self.calls]).reshape(-1, 12),
+                                            np.concatenate([c[3] for c in self.calls] + [np.zeros(0, np.uint8)]),
+                                            np.cumsum([0] + [len(c[3]) for c in self.calls])))
+        else:
+            assert self.mismatch is None, f"essential-matrix call {self.mismatch} is not the recorded reference's call"
+            assert len(self.calls) == len(self.want[1]), (len(self.calls), len(self.want[1]))
+
+
+def reference_system_trace(ref_results, key, seq, K, world_points=True):
+    """The reference's own System over the host RGBA frames `seq` (run live, or as recorded): per frame (status, info8, Twc,
+    ids, 3-D flags, digest of the pixel positions, world points -- empty unless `world_points`)."""
+    h, w = seq[0].shape[:2]
+
+    def run_reference():
+        ref = ref_results.lib
+        ref.ref_system_create.restype = C.c_void_p
+        ref.ref_system_create.argtypes = [C.c_int, C.c_int] + [C.c_double] * 8
+        ref.ref_system_find_camera_pose.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]
+        ref.ref_system_keypoints.argtypes = [C.c_void_p] * 5 + [C.c_int, C.c_void_p]
+        ref.ref_system_info8.argtypes = [C.c_void_p, C.c_void_p]
+        ref.ref_system_destroy.argtypes = [C.c_void_p]
+        r = ref.ref_system_create(w, h, K[0], K[1], K[2], K[3], 0, 0, 0, 0)
+        st, info, T, frames = [], [], [], []
+        for k, f in enumerate(seq):
+            pose = np.zeros(16, np.float32); T_r = np.zeros(7); i_r = np.zeros(8, np.int32)
+            st.append(ref.ref_system_find_camera_pose(r, P(np.ascontiguousarray(f)), k * 33.333, P(pose)))
+            ids_r = np.zeros(CAP, np.int32); px_r = np.zeros((CAP, 2), np.float32); d3_r = np.zeros(CAP, np.uint8); w_r = np.zeros((CAP, 3))
+            n_r = ref.ref_system_keypoints(r, P(ids_r), P(px_r), P(d3_r), P(w_r), CAP, P(T_r))
+            ref.ref_system_info8(r, P(i_r))
+            info.append(i_r); T.append(T_r); frames.append((ids_r[:n_r], d3_r[:n_r], px_r[:n_r], w_r[:n_r if world_points else 0]))
+        ref.ref_system_destroy(r)
+        return (np.array(st, np.int32), np.array(info), np.array(T), np.cumsum([0] + [len(f[0]) for f in frames]),
+                np.concatenate([f[0] for f in frames]), np.concatenate([f[1] for f in frames]), np.array([digest(f[2]) for f in frames]),
+                np.cumsum([0] + [len(f[3]) for f in frames]), np.concatenate([f[3] for f in frames]))
+    st, info, T, start, ids, d3, px, wstart, wp = ref_results.get(key, run_reference)
+    return [(int(st[k]), info[k], T[k], ids[start[k]:start[k + 1]], d3[start[k]:start[k + 1]], px[k], wp[wstart[k]:wstart[k + 1]])
+            for k in range(len(seq))]
 
 
 def quat_dist(a, b):

@@ -1,5 +1,5 @@
 """CPU tests: the detector oracle (oracle/detect_oracle.c) against (a) golden vectors dumped from the reference's own
-FeatureExtractor (tools/make_golden_detect.py) and (b) the live reference when it is built here.  Bit-exact, floats included."""
+FeatureExtractor (tools/make_golden_detect.py) and (b) the reference, live or recorded.  Bit-exact, floats included."""
 import ctypes as C
 
 import numpy as np
@@ -32,17 +32,19 @@ def test_detect_golden(oracle, tag):
 
 
 @pytest.mark.parametrize("w,h,cs,seed,ncur", [(640, 480, 40, 5, 0), (640, 480, 40, 6, 80), (1280, 720, 40, 7, 250), (400, 300, 30, 8, 20)])
-def test_detect_live_reference(oracle, ref, w, h, cs, seed, ncur):
-    if ref is None or not hasattr(ref, "ref_detect_points"):
-        pytest.skip("oracle/_ref/libalva_ref.so (with FeatureExtractor) not built in this tree")
+def test_detect_live_reference(oracle, ref_results, w, h, cs, seed, ncur):
     fr, _ = synth.make_frames(1, w, h, seed=seed, rgba=False)
     img = np.ascontiguousarray(fr[0])
     cur = random_cur(w, h, ncur, seed)
     roi = np.array([20, 20, w - 40, h - 40], np.int32)
-    ref.ref_detect_points.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_double, C.c_void_p, C.c_int]
     for q0 in (0.001, 0.00002):
-        want = np.zeros((4096, 2), np.float32)
-        n = ref.ref_detect_points(P(img), w, h, cs, P(cur), ncur, P(roi), q0, P(want), 4096)
+        def detect():
+            ref = ref_results.lib
+            ref.ref_detect_points.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_double, C.c_void_p, C.c_int]
+            want = np.zeros((4096, 2), np.float32)
+            n = ref.ref_detect_points(P(img), w, h, cs, P(cur), ncur, P(roi), q0, P(want), 4096)
+            return (n, want[:n])
+        n, want = ref_results.get(f"detect/{w}x{h}/{cs}/{seed}/{ncur}/{q0}", detect)
         pts, _, _ = oracle_detect(oracle, img, cs, cur, roi, q0)
         assert len(pts) == n
         assert (bits(pts) == bits(want[:n])).all()
@@ -70,19 +72,23 @@ def test_occupied_cells_are_skipped(oracle):
     assert d.min() > 9.0   # nothing inside the radius-10 discs
 
 
-def test_corner_subpix_live_reference_with_border_points(oracle, ref):
+def test_corner_subpix_live_reference_with_border_points(oracle, ref_results):
     """cv::cornerSubPix incl. the replicate-border sampling path (points within 5 px of the frame)."""
-    if ref is None or not hasattr(ref, "ref_corner_subpix"):
-        pytest.skip("oracle/_ref/libalva_ref.so not built in this tree")
     w, h, n = 320, 240, 600
     fr, _ = synth.make_frames(1, w, h, seed=4, rgba=False)
     img = np.ascontiguousarray(fr[0])
     rng = np.random.default_rng(2)
     pts = np.stack([rng.uniform(0, w - 1, n), rng.uniform(0, h - 1, n)], 1).astype(np.float32)
     pts[:50, 0] = rng.uniform(0, 5, 50); pts[50:100, 1] = rng.uniform(h - 6, h - 1, 50); pts[100:150, 0] = rng.uniform(w - 6, w - 1, 50)
-    a, b = pts.copy(), pts.copy()
-    ref.ref_corner_subpix.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_double]
-    oracle.orc_corner_subpix.argtypes = ref.ref_corner_subpix.argtypes
-    ref.ref_corner_subpix(P(img), w, h, P(a), n, 3, 30, 0.01)
+    args = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_double]
+
+    def subpix():
+        a = pts.copy()
+        ref_results.lib.ref_corner_subpix.argtypes = args
+        ref_results.lib.ref_corner_subpix(P(img), w, h, P(a), n, 3, 30, 0.01)
+        return (a,)
+    a, = ref_results.get("corner_subpix", subpix)
+    b = pts.copy()
+    oracle.orc_corner_subpix.argtypes = args
     oracle.orc_corner_subpix(P(img), w, h, P(b), n, 3, 30, 0.01)
     assert (bits(a) == bits(b)).all()

@@ -1,5 +1,5 @@
 """CPU tests: the KLT oracle (oracle/klt_oracle.c) against (a) golden vectors dumped from the reference's own
-FeatureTracker + vendored OpenCV 4.5.5 (tools/make_golden_klt.py) and (b) the live reference when it exists in this tree.
+FeatureTracker + vendored OpenCV 4.5.5 (tools/make_golden_klt.py) and (b) the reference, live or recorded.
 Bit-exact: positions are compared as float bit patterns."""
 import ctypes as C
 
@@ -44,21 +44,23 @@ def test_klt_lk_golden(oracle, levels, ui):
 
 
 @pytest.mark.parametrize("w,h,seed", [(161, 91, 2), (320, 240, 7)])
-def test_fb_klt_live_reference(oracle, ref, w, h, seed):
-    if ref is None:
-        pytest.skip("oracle/_ref/libalva_ref.so not built in this tree")
+def test_fb_klt_live_reference(oracle, ref_results, w, h, seed):
+    ref = ref_results.lib
     fr, _ = synth.make_frames(2, w, h, seed=seed, rgba=False)
     a, b = np.ascontiguousarray(fr[0]), np.ascontiguousarray(fr[1])
     n = 250
     pts, pri = klt_points(w, h, n, seed)
-    L = ref.ref_build_pyramid(P(a), w, h, 9, 3, None, None)
+    L = int(ref_results.get(f"pyramid_levels/{w}x{h}/{seed}", lambda: (ref.ref_build_pyramid(P(a), w, h, 9, 3, None, None),))[0])
     pa, da = build_pyramid(oracle, a, L)
     pb, db = build_pyramid(oracle, b, L)
-    ref.ref_fb_klt.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float,
-                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
     for levels in (1, 3):
-        q1, g1 = pri.copy(), np.zeros(n, np.uint8)
-        ref.ref_fb_klt(P(a), P(b), w, h, 9, 3, levels, 30.0, 0.5, P(pts), P(q1), P(g1), n)
+        def fb_klt():
+            ref.ref_fb_klt.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
+            q1, g1 = pri.copy(), np.zeros(n, np.uint8)
+            ref.ref_fb_klt(P(a), P(b), w, h, 9, 3, levels, 30.0, 0.5, P(pts), P(q1), P(g1), n)
+            return (q1, g1)
+        q1, g1 = ref_results.get(f"fb_klt/{w}x{h}/{seed}/{levels}", fb_klt)
         q2, g2 = oracle_fb_klt(oracle, pa, da, pb, db, w, h, levels, pts, pri)
         assert (g1 == g2).all() and g1.sum() > 50
         assert (bits(q1) == bits(q2)).all()

@@ -1,5 +1,5 @@
 """CPU tests: the matchToMap oracle (oracle/match_oracle.c) against (a) golden vectors dumped from the reference's own Mapper
-(tools/make_golden_match.py) and (b) the live reference when it is built here.  Exact: identical keypoint -> map point maps."""
+(tools/make_golden_match.py) and (b) the reference, live or recorded.  Exact: identical keypoint -> map point maps."""
 import numpy as np
 import pytest
 
@@ -30,12 +30,14 @@ def test_match_golden(oracle, seed, nkp3d):
 
 
 @pytest.mark.parametrize("seed", [11, 12, 13, 14, 15, 16])
-def test_match_live_reference(oracle, ref, seed):
-    if ref is None or not hasattr(ref, "ref_match_to_map"):
-        pytest.skip("oracle/_ref/libalva_ref.so (full AlvaAR build) not present in this tree")
+def test_match_live_reference(oracle, ref_results, seed):
     p = synth.make_match_problem(seed, n_frame_kp=120 + 13 * (seed % 5), n_local=300 + 37 * (seed % 7), dup_frac=0.5)
     for nk in (100, 5):
-        order, want = reference_match(ref, p, nk)
+        def match():
+            order, m = reference_match(ref_results.lib, p, nk)
+            return (order, np.array(sorted(m.items()), np.int32).reshape(-1, 2))
+        order, want = ref_results.get(f"match/{seed}/{nk}", match)
+        want = dict(want.tolist())
         assert oracle_match(oracle, p, order, nk) == want and len(want) > 30
 
 

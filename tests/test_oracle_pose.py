@@ -1,5 +1,5 @@
 """CPU tests: the pose oracle (oracle/pose_oracle.c) against (a) golden vectors dumped from the reference's own
-MultiViewGeometry + vendored OpenGV / Ceres (tools/make_golden_pose.py) and (b) the live reference when it is built here.
+MultiViewGeometry + vendored OpenGV / Ceres (tools/make_golden_pose.py) and (b) the reference, live or recorded.
 fp64: poses within 1e-9 (far inside the 1e-4 relative bar), inlier / outlier sets exact."""
 import ctypes as C
 
@@ -69,20 +69,26 @@ def test_sampler_sequence_is_mt19937_shift(oracle):
 
 
 @pytest.mark.parametrize("n,seed,of", [(120, 11, 0.2), (700, 12, 0.35), (9, 13, 0.0)])
-def test_pose_live_reference(oracle, ref, n, seed, of):
-    if ref is None or not hasattr(ref, "ref_p3p_lmeds"):
-        pytest.skip("oracle/_ref/libalva_ref.so (with OpenGV) not built in this tree")
+def test_pose_live_reference(oracle, ref_results, n, seed, of):
+    ref = ref_results.lib
     pr = make_pose_problem(n, seed, outlier_frac=of)
     K32 = pr["K"].astype(np.float32)
-    ref.ref_p3p_lmeds.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, f32, f32, f32, C.c_void_p, C.c_void_p]
-    ref.ref_pnp.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, f32, C.c_int, C.c_int, f32, f32, f32, f32, C.c_void_p]
-    T1, o1 = np.zeros(12), np.zeros(n, np.uint8)
-    ok1 = ref.ref_p3p_lmeds(P(pr["bv"]), P(pr["X"]), n, 100, 3.0, K32[0], K32[1], P(T1), P(o1))
+
+    def p3p():
+        ref.ref_p3p_lmeds.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, f32, f32, f32, C.c_void_p, C.c_void_p]
+        T1, o1 = np.zeros(12), np.zeros(n, np.uint8)
+        ok1 = ref.ref_p3p_lmeds(P(pr["bv"]), P(pr["X"]), n, 100, 3.0, K32[0], K32[1], P(T1), P(o1))
+        return (ok1, T1, o1)
+    ok1, T1, o1 = ref_results.get(f"p3p/{n}/{seed}/{of}", p3p)
     ok2, T2, o2, _ = orc_p3p(oracle, pr["bv"], pr["X"], K32)
     assert ok1 == ok2 == 1 and (o1 == o2).all() and np.abs(T1 - T2).max() < 1e-9
     for rob, l2 in ((1, 1), (0, 0)):
-        p1, oo1 = pr["pose0"].copy(), np.zeros(n, np.uint8)
-        k1 = ref.ref_pnp(P(pr["uv"]), P(pr["X"]), n, P(p1), 5, 5.9915, rob, l2, K32[0], K32[1], K32[2], K32[3], P(oo1))
+        def pnp():
+            ref.ref_pnp.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, f32, C.c_int, C.c_int, f32, f32, f32, f32, C.c_void_p]
+            p1, oo1 = pr["pose0"].copy(), np.zeros(n, np.uint8)
+            k1 = ref.ref_pnp(P(pr["uv"]), P(pr["X"]), n, P(p1), 5, 5.9915, rob, l2, K32[0], K32[1], K32[2], K32[3], P(oo1))
+            return (k1, p1, oo1)
+        k1, p1, oo1 = ref_results.get(f"pnp/{n}/{seed}/{of}/{rob}{l2}", pnp)
         k2, p2, oo2, _ = orc_pnp(oracle, pr["uv"], pr["X"], K32.astype(np.float64), pr["pose0"], rob, l2)
         assert k1 == k2 == 1 and (oo1 == oo2).all() and np.abs(p1 - p2).max() < 1e-9
 

@@ -10,17 +10,17 @@ What is toleranced: after the initialisation, poses / world points carry the ref
 (tests/test_oracle_init.py: a 1-ulp input change moves ITS result by 1e-6 .. 1e-3).  The bar is data-driven (system_util.
 pose_deviation): 1e-4 relative (north_star), or 4 x the reference's OWN spread on this trace under a 1-ulp change of one intrinsic
 (stored in the golden) where that spread is larger; the worst observed deviation is printed.
-With the reference's OWN initialisation stage plugged in (live reference only) everything downstream -- KLT with projected
+With the reference's OWN initialisation stage plugged in (live, or its recorded results) everything downstream -- KLT with projected
 priors, P3P-LMedS, PnP, keyframe decisions, triangulation, local-map matching, local BA, culling -- is in lockstep: poses and
 world points 1e-9, pixel positions bit-identical, over the whole trace (tools/compare_system_cpu.py shows the same over 140
 frames / 11 keyframes / 9 local BAs)."""
 import ctypes as C
 
 import numpy as np
-import pytest
 
-from conftest import P
-from system_util import CAP, PoseReport, cpu_system_lib, frame_slice, frames_and_golden, quat_dist
+from conftest import P, digest
+from system_util import (CAP, PoseReport, ReferenceEssential, cpu_system_lib, frame_slice, frames_and_golden, quat_dist,
+                         reference_system_trace)
 
 
 def run(S, frames, K, hook=None):
@@ -64,11 +64,11 @@ def test_state_machine_follows_the_reference(oracle):
     rep.summary(g)
 
 
-def test_lockstep_given_the_reference_initialisation(oracle, ref):
-    if ref is None:
-        pytest.skip("oracle/_ref not built here")
+def test_lockstep_given_the_reference_initialisation(oracle, ref_results):
     g, frames = frames_and_golden()
-    tr = run(cpu_system_lib(), frames, g["K"], C.cast(ref.ref_essential_5pt, C.c_void_p))
+    hook = ReferenceEssential(ref_results, "lockstep/essential")
+    tr = run(cpu_system_lib(), frames, g["K"], hook.ptr)
+    hook.finish()
     assert int(g["first_ba_frame"]) < len(frames) - 5                        # the trace does contain a local BA
     for k in range(len(frames)):
         st, T, info, ids, px, d3, wp = tr[k]
@@ -100,12 +100,40 @@ def test_reset_when_tracks_are_lost(oracle):
     S.cpu_system_destroy(s)
 
 
-def test_failure_paths_in_lockstep_with_the_live_reference(oracle, ref):
+def lockstep_with_reference_system(ref_results, key, seq, K, pose_tol, wpt_tol=None):
+    """The state machine over the CPU oracle, the reference's own initialisation stage plugged in, frame by frame against the
+    reference's own System: every discrete quantity equal, pixel positions bit-identical, poses (and world points) to the
+    given bars.  Returns the reference's trace."""
+    h, w = seq[0].shape[:2]
+    want = reference_system_trace(ref_results, key + "/system", seq, K, world_points=wpt_tol is not None)
+    S = cpu_system_lib()
+    s = S.cpu_system_create(w, h, K[0], K[1], K[2], K[3])
+    hook = ReferenceEssential(ref_results, key + "/essential")
+    S.cpu_system_set_essential_hook(s, hook.ptr)
+    for k, f in enumerate(seq):
+        T_s = np.zeros(7)
+        st_s = S.cpu_system_process(s, P(np.ascontiguousarray(f)), k * 33.333, P(T_s))
+        ids_s = np.zeros(CAP, np.int32); px_s = np.zeros((CAP, 2), np.float32); d3_s = np.zeros(CAP, np.uint8); w_s = np.zeros((CAP, 3))
+        n_s = S.cpu_system_keypoints(s, P(ids_s), P(px_s), P(d3_s), P(w_s), CAP)
+        i_s = np.zeros(8, np.int32)
+        S.cpu_system_info(s, P(i_s))
+        st_r, i_r, T_r, ids_r, d3_r, px_r, w_r = want[k]
+        n_r = len(ids_r)
+        assert st_r == st_s and n_r == n_s and (i_r == i_s).all(), (k, st_r, st_s, i_r, i_s)
+        assert (ids_r == ids_s[:n_s]).all() and (d3_r == d3_s[:n_s]).all(), k
+        assert (digest(px_s[:n_s]) == px_r).all(), k                       # bit-identical pixel positions
+        assert np.abs(T_r - T_s).max() < pose_tol, k
+        if wpt_tol is not None:
+            assert np.abs(w_r - w_s[:n_s]).max() < wpt_tol * max(1.0, np.abs(w_r).max()), k
+    S.cpu_system_destroy(s)
+    hook.finish()
+    return want
+
+
+def test_failure_paths_in_lockstep_with_the_live_reference(oracle, ref_results):
     """Blackout frame, a jump to an unrelated sequence, a jump back: lost tracks, P3P / PnP outlier removal, failed poses,
-    resets (status 2) with a stale motion model, re-initialisations -- against the live reference System frame by frame
+    resets (status 2) with a stale motion model, re-initialisations -- against the reference System frame by frame
     (its own initialisation stage plugged in): every discrete quantity equal, poses 1e-6."""
-    if ref is None:
-        pytest.skip("oracle/_ref not built here")
     from alvaar_b200 import synth
     w, h = 640, 480
     K = synth.intrinsics(w, h)
@@ -113,77 +141,19 @@ def test_failure_paths_in_lockstep_with_the_live_reference(oracle, ref):
     B, _ = synth.make_frames(26, w, h, seed=33, rgba=True)
     black = np.zeros_like(A[0]); black[..., 3] = 255
     seq = [A[k] for k in range(24)] + [black] + [B[k] for k in range(26)] + [A[k] for k in range(20, 40)]
-    ref.ref_system_create.restype = C.c_void_p
-    ref.ref_system_create.argtypes = [C.c_int, C.c_int] + [C.c_double] * 8
-    ref.ref_system_find_camera_pose.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]
-    ref.ref_system_keypoints.argtypes = [C.c_void_p] * 5 + [C.c_int, C.c_void_p]
-    ref.ref_system_info8.argtypes = [C.c_void_p, C.c_void_p]
-    ref.ref_system_destroy.argtypes = [C.c_void_p]
-    S = cpu_system_lib()
-    r = ref.ref_system_create(w, h, K[0], K[1], K[2], K[3], 0, 0, 0, 0)
-    s = S.cpu_system_create(w, h, K[0], K[1], K[2], K[3])
-    S.cpu_system_set_essential_hook(s, C.cast(ref.ref_essential_5pt, C.c_void_p))
-    seen = set()
-    for k, f in enumerate(seq):
-        f = np.ascontiguousarray(f)
-        pose = np.zeros(16, np.float32); T_s = np.zeros(7); T_r = np.zeros(7)
-        st_r = ref.ref_system_find_camera_pose(r, P(f), k * 33.333, P(pose))
-        st_s = S.cpu_system_process(s, P(f), k * 33.333, P(T_s))
-        ids_r = np.zeros(CAP, np.int32); px_r = np.zeros((CAP, 2), np.float32); d3_r = np.zeros(CAP, np.uint8); w_r = np.zeros((CAP, 3))
-        ids_s = np.zeros(CAP, np.int32); px_s = np.zeros((CAP, 2), np.float32); d3_s = np.zeros(CAP, np.uint8); w_s = np.zeros((CAP, 3))
-        n_r = ref.ref_system_keypoints(r, P(ids_r), P(px_r), P(d3_r), P(w_r), CAP, P(T_r))
-        n_s = S.cpu_system_keypoints(s, P(ids_s), P(px_s), P(d3_s), P(w_s), CAP)
-        i_r = np.zeros(8, np.int32); i_s = np.zeros(8, np.int32)
-        ref.ref_system_info8(r, P(i_r)); S.cpu_system_info(s, P(i_s))
-        assert st_r == st_s and n_r == n_s and (i_r == i_s).all(), (k, st_r, st_s, i_r, i_s)
-        assert (ids_r[:n_r] == ids_s[:n_s]).all() and (d3_r[:n_r] == d3_s[:n_s]).all(), k
-        assert (px_r[:n_r].view(np.uint32) == px_s[:n_s].view(np.uint32)).all(), k
-        assert np.abs(T_r - T_s).max() < 1e-6, k
-        seen.add(st_r)
-    assert seen == {1, 2, 3}                                              # the sequence did exercise resets and re-initialisation
-    ref.ref_system_destroy(r)
-    S.cpu_system_destroy(s)
+    want = lockstep_with_reference_system(ref_results, "failure_paths", seq, K, 1e-6)
+    assert {f[0] for f in want} == {1, 2, 3}                              # the sequence did exercise resets and re-initialisation
 
 
-def test_lockstep_at_720p_with_the_live_reference(oracle, ref):
+def test_lockstep_at_720p_with_the_live_reference(oracle, ref_results):
     """BASELINE's frame size (1280x720, 784 keypoints / frame): 36 frames through initialisation (frame 12), two more keyframes
-    and the first local BA against the live reference System, its own initialisation stage plugged in: lockstep as at 640x480."""
-    if ref is None:
-        pytest.skip("oracle/_ref not built here")
+    and the first local BA against the reference System, its own initialisation stage plugged in: lockstep as at 640x480."""
     from alvaar_b200 import synth
     w, h, nf = 1280, 720, 36
     K = synth.intrinsics(w, h)
     frames, _ = synth.make_frames(nf, w, h, seed=7, rgba=True)
-    ref.ref_system_create.restype = C.c_void_p
-    ref.ref_system_create.argtypes = [C.c_int, C.c_int] + [C.c_double] * 8
-    ref.ref_system_find_camera_pose.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]
-    ref.ref_system_keypoints.argtypes = [C.c_void_p] * 5 + [C.c_int, C.c_void_p]
-    ref.ref_system_info8.argtypes = [C.c_void_p, C.c_void_p]
-    ref.ref_system_destroy.argtypes = [C.c_void_p]
-    S = cpu_system_lib()
-    r = ref.ref_system_create(w, h, K[0], K[1], K[2], K[3], 0, 0, 0, 0)
-    s = S.cpu_system_create(w, h, K[0], K[1], K[2], K[3])
-    S.cpu_system_set_essential_hook(s, C.cast(ref.ref_essential_5pt, C.c_void_p))
-    last = None
-    for k in range(nf):
-        f = np.ascontiguousarray(frames[k])
-        pose = np.zeros(16, np.float32); T_s = np.zeros(7); T_r = np.zeros(7)
-        st_r = ref.ref_system_find_camera_pose(r, P(f), k * 33.333, P(pose))
-        st_s = S.cpu_system_process(s, P(f), k * 33.333, P(T_s))
-        ids_r = np.zeros(CAP, np.int32); px_r = np.zeros((CAP, 2), np.float32); d3_r = np.zeros(CAP, np.uint8); w_r = np.zeros((CAP, 3))
-        ids_s = np.zeros(CAP, np.int32); px_s = np.zeros((CAP, 2), np.float32); d3_s = np.zeros(CAP, np.uint8); w_s = np.zeros((CAP, 3))
-        n_r = ref.ref_system_keypoints(r, P(ids_r), P(px_r), P(d3_r), P(w_r), CAP, P(T_r))
-        n_s = S.cpu_system_keypoints(s, P(ids_s), P(px_s), P(d3_s), P(w_s), CAP)
-        i_r = np.zeros(8, np.int32); i_s = np.zeros(8, np.int32)
-        ref.ref_system_info8(r, P(i_r)); S.cpu_system_info(s, P(i_s))
-        assert st_r == st_s and n_r == n_s and (i_r == i_s).all(), (k, st_r, st_s, i_r, i_s)
-        assert (ids_r[:n_r] == ids_s[:n_s]).all() and (d3_r[:n_r] == d3_s[:n_s]).all(), k
-        assert (px_r[:n_r].view(np.uint32) == px_s[:n_s].view(np.uint32)).all(), k
-        assert np.abs(T_r - T_s).max() < 1e-9 and np.abs(w_r[:n_r] - w_s[:n_s]).max() < 1e-9 * max(1.0, np.abs(w_r[:n_r]).max()), k
-        last = i_r
+    last = lockstep_with_reference_system(ref_results, "720p", [frames[k] for k in range(nf)], K, 1e-9, 1e-9)[-1][1]
     assert last[4] == 1 and last[1] >= 2 and last[2] > 500          # initialised, at least keyframe 2 (a local BA ran), 720p-sized
-    ref.ref_system_destroy(r)
-    S.cpu_system_destroy(s)
 
 
 def test_find_plane_on_the_planar_scene(oracle):
